@@ -251,6 +251,36 @@ def _roofline(pipe, stage_ms, ms_step, workload, pairs):
     return roof, roof_path
 
 
+DUMP_GAUSSIANS = 1 << 16   # Gaussians whose gradients --dump-outputs keeps
+DUMP_PIXELS = 1 << 21      # pixels it keeps of a larger image: a dump stays below 64 MB at every workload
+
+
+def _dump_rows(t, k):
+    """Rows of t at a fixed, seeded set of k indices; all of t when it has no more than k rows."""
+    import numpy as np
+    import torch
+    if t.shape[0] <= k:
+        return t
+    rows = np.sort(np.random.default_rng(0).choice(t.shape[0], size=k, replace=False))
+    return t.index_select(0, torch.from_numpy(rows).to(t.device))
+
+
+def dump_outputs(out_dir, pipe):
+    """Writes what the timed step hands its caller -- the rendered image, the loss and the gradient of every Gaussian
+    parameter -- as float32 DIR/<name>.npy, so that two builds can be compared output for output.  The gradients are
+    kept for DUMP_GAUSSIANS Gaussians, an image of more than DUMP_PIXELS pixels for that many (as [k, 3]); both
+    samples are the same rows in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    img = pipe.out_img
+    if img.shape[0] * img.shape[1] > DUMP_PIXELS:
+        img = _dump_rows(img.reshape(-1, 3), DUMP_PIXELS)
+    arrays = {"image": img, "loss": pipe.loss}
+    arrays.update({"grad_" + k: _dump_rows(v, DUMP_GAUSSIANS) for k, v in pipe.g.items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def _side_config(workload, dev, steps=5, warmup=3):
     """One-shot sub-record for another BASELINE config (C3 / C5) on this GPU: value, stages, roofline."""
     import torch
@@ -368,6 +398,8 @@ def run_ours(args):
     # the headline region: K steps, no instrumentation between the kernels
     pipe.stage_timing = False
     ms_total = timed(step_fwd_bwd, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pipe)
     # the same K steps again with a CUDA event at every stage boundary (stage times, roofline): the ~20 timing events
     # per step cost 1-2 % (each one drains the launch pipeline for a moment), which is why they are not in the
     # headline region; `ms_per_step_instrumented` says what the step took with them
@@ -512,7 +544,7 @@ def run_ours(args):
         del P, gflat
         for wl in ("c3_3M_4k_sh3", "c5_5M_1440p_dense"):
             try:
-                side[wl] = _side_config(wl, dev)
+                side[wl] = _side_config(wl, dev, steps=args.steps, warmup=max(args.warmup, 3))
             except Exception as ex:   # a sub-record must never cost the headline line
                 side[wl] = {"error": str(ex)[:300]}
 
@@ -581,7 +613,7 @@ if __name__ == "__main__":
     _watchdog(1500)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every measured region (>= 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2_1M_1080p_sh3", choices=list(WORKLOADS))
@@ -592,7 +624,13 @@ if __name__ == "__main__":
     ap.add_argument("--exchange", default="fused", choices=["fused", "nccl"],
                     help="N>1: fused multi-view SH backward + all-reduce launch over peer memory (default) or plain "
                          "NCCL all-reduce of the flat gradient buffer")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (image, loss, sampled gradients) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     if a.impl == "reference":
         run_reference(a)
     else:

@@ -70,5 +70,28 @@ def build(force=False):
     return OUT
 
 
+TEST_SRC = os.path.join(HERE, "..", "tests", "native", "model_forward_op.cpp")
+TEST_OUT = os.path.join(HERE, "..", "tests", "native", "_build", "libopensplat_b200_test_ops.so")
+
+
+def build_test_ops(force=False):
+    """Test-only binding of gsb::modelForward (tests/native/model_forward_op.cpp) ->
+    tests/native/_build/libopensplat_b200_test_ops.so, linked against the operator library built above."""
+    build()
+    if not force and os.path.exists(TEST_OUT) and all(
+            os.path.getmtime(d) <= os.path.getmtime(TEST_OUT) for d in (TEST_SRC, OUT)):
+        return TEST_OUT
+    os.makedirs(os.path.dirname(TEST_OUT), exist_ok=True)
+    lib_dir = os.path.join(HERE, "lib")
+    cmd = [CXX] + FLAGS + ["-shared", TEST_SRC, "-o", TEST_OUT] + shared_stdcxx_flags() + [
+        f"-L{lib_dir}", "-lopensplat_b200_ops", "-lgsplat_b200", "-Wl,-rpath,$ORIGIN/../../../opensplat_b200/lib",
+        f"-L{TORCH}/lib", f"-Wl,-rpath,{TORCH}/lib", "-ltorch", "-ltorch_cpu", "-ltorch_cuda", "-lc10", "-lc10_cuda",
+        "-L/usr/local/cuda/lib64", "-lcudart"]
+    r = subprocess.run(cmd, capture_output=True, text=True)
+    if r.returncode != 0:
+        raise RuntimeError(f"test ops build failed:\n{r.stderr[-4000:]}")
+    return TEST_OUT
+
+
 if __name__ == "__main__":
     print(build(force="--force" in sys.argv))

@@ -2,7 +2,7 @@
 // reference's simple_trainer.cpp:26-62 uses (Options, add_options()(...) chains, value<T>()->default_value,
 // parse, count, operator[]().as<T>(), help).  cxxopts itself is a FetchContent dependency of the
 // reference (CMakeLists.txt) that is not available offline; this shim exists ONLY so that the unchanged
-// simple_trainer.cpp can be compiled against the gsplat_b200 operator layer (tools/build_simple_trainer.py).
+// simple_trainer.cpp can be compiled against the gsplat_b200 operator layer (oracle/build_simple_trainer.py).
 #pragma once
 #include <map>
 #include <memory>

@@ -1,8 +1,8 @@
 // tests/native/model_driver.cpp -- TEST INFRASTRUCTURE ONLY.
-// Drives the UNMODIFIED reference Model (model.cpp compiled from /root/reference).  Built twice:
+// Drives the UNMODIFIED reference Model (model.cpp compiled from the reference tree).  Built twice:
 //  (1) oracle/Makefile -> oracle/_ref/libopensplat_ref_model.so: model.cpp + the reference's own CPU operators; pins the
 //      restatements in oracle/scene_edit.py against the reference itself (torch.ops.opensplat_ref_model.*);
-//  (2) tools/build_model_b200.py -> opensplat_b200/lib/libopensplat_model_b200.so: the SAME unmodified model.cpp compiled
+//  (2) oracle/build_model_b200.py -> oracle/_ref/libopensplat_model_b200.so: the SAME unmodified model.cpp compiled
 //      with -DUSE_CUDA against THIS repo's operator layer (csrc/ops) -- the drop-in check that Model::forward /
 //      mainLoss / optimizersStep / afterTrain run unchanged on the B200 back end (torch.ops.opensplat_b200_model.*).
 //   after_train   -> Model::afterTrain  (model.cpp:311-500), incl. the Adam-state surgery

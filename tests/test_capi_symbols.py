@@ -58,7 +58,7 @@ def test_cxx_libraries_use_the_shared_libstdcxx():
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     libs = [os.path.join(root, "opensplat_b200", "lib", "libopensplat_b200_ops.so"),
-            os.path.join(root, "tests", "native", "_build", "libopensplat_model_b200.so"),
+            os.path.join(root, "oracle", "_ref", "libopensplat_model_b200.so"),
             os.path.join(root, "oracle", "_ref", "libopensplat_ref_cpu.so"),
             os.path.join(root, "oracle", "_ref", "libopensplat_ref_model.so")]
     checked = 0

@@ -1,133 +1,125 @@
 """Drop-in check for the real caller of the hot path: the reference's model.cpp compiled UNCHANGED (-DUSE_CUDA)
-against this repo's operator layer (tools/build_model_b200.py -> libopensplat_model_b200.so) runs the body of the
+against this repo's operator layer (oracle/build_model_b200.py -> libopensplat_model_b200.so) runs the body of the
 reference training loop (opensplat.cpp:151-170: forward, mainLoss, backward, optimizersStep, schedulersStep,
-afterTrain incl. two densifications) on the B200 back end, and the host-side mirror opensplat_b200.model.GaussianModel
-(fused activations / loss / Adam / topology edits) follows the same trajectory.
+afterTrain incl. two densifications) on the B200 back end.  What that run computes -- the reference's caller over THIS
+repo's operators, so a regression baseline of this project rather than an output of the reference alone -- is stored
+in tests/golden/b200_model_train.npz (tests/golden/make_golden_b200.py).  The host-side mirror
+opensplat_b200.model.GaussianModel (fused activations / loss / Adam / topology edits) follows the same trajectory.
 
 Both sides use the same CUDA kernels for the three operators; what differs is everything around them (ATen ops in
 the reference's Model vs the fused kernels), so agreement is to round-off until the first refinement and, because a
 refinement takes discrete decisions on values that differ in the last bits, to a looser bound afterwards."""
 import os
 import sys
+import types
 
 import numpy as np
 import pytest
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from util import PARAM_NAMES  # noqa: E402
+from util import (PARAM_NAMES, TRAIN_REFINE, TRAIN_SEED, TRAIN_SH_INTERVAL, TRAIN_SSIM_WEIGHT,  # noqa: E402
+                  TRAIN_STEPS, load_golden, make_problem)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "tests", "native", "_build", "libopensplat_model_b200.so")
 
 
-def make_problem(n=4000, V=3, H=96, W=128, k=4, seed=5):
-    rng = np.random.default_rng(seed)
-    f = np.float32
-    p = {
-        "means": (rng.uniform(-1, 1, (n, 3)) * np.array([1.6, 1.2, 0.5])).astype(f),
-        "scales": np.log(rng.uniform(0.02, 0.12, (n, 3))).astype(f),
-        "quats": rng.standard_normal((n, 4)).astype(f),
-        "featuresDc": rng.uniform(-1.5, 1.5, (n, 3)).astype(f),
-        "featuresRest": (rng.standard_normal((n, k - 1, 3)) * 0.1).astype(f),
-        "opacities": rng.uniform(-2.0, 1.0, (n, 1)).astype(f),
-    }
-    c2w = np.tile(np.eye(4, dtype=f), (V, 1, 1))
-    for v in range(V):                       # OpenGL-style poses on a circle of radius 4, looking at the origin
-        a = 0.25 * (v - (V - 1) / 2)
-        c2w[v, :3, :3] = np.array([[np.cos(a), 0, -np.sin(a)], [0, 1, 0], [np.sin(a), 0, np.cos(a)]], dtype=f)
-        c2w[v, :3, 3] = np.array([-4.0 * np.sin(a), 0.0, 4.0 * np.cos(a)], dtype=f)
-    yy, xx = np.mgrid[0:H, 0:W]
-    gts = np.stack([np.stack([0.5 + 0.5 * np.sin(0.07 * xx + v), 0.5 + 0.5 * np.cos(0.05 * yy - v),
-                              0.5 + 0.25 * np.sin(0.03 * (xx + yy))], -1) for v in range(V)]).astype(f)
-    return p, c2w, gts, (0.9 * W, 0.9 * W, W / 2.0, H / 2.0), H, W
+def _reference_run():
+    """The reference's training loop on the B200 operators (golden): losses, counts, last image and the parameters
+    at the stored rows."""
+    g = load_golden("b200_model_train")
+    ref_loss, ref_cnt = g["loss"], g["count"]
+    assert np.isfinite(ref_loss).all() and ref_loss[18] < ref_loss[0]            # it trains
+    assert ref_cnt[18] == len(make_problem()[0]["means"])
+    assert ref_cnt[19] != ref_cnt[18] and ref_cnt[29] != ref_cnt[28]              # two refinements happened
+    rows = torch.from_numpy(g["param_rows"]).to(DEV)
+    return (ref_loss, ref_cnt, torch.from_numpy(g["rgb"]).to(DEV),
+            {k: torch.from_numpy(g[k]).to(DEV) for k in PARAM_NAMES}, rows)
 
 
-@pytest.mark.skipif(not os.path.exists(LIB), reason="libopensplat_model_b200.so not built (needs /root/reference at build time)")
-def test_reference_model_cpp_unchanged_trains_on_b200_backend_and_mirror_follows():
-    from opensplat_b200 import cpp_ops
-    cpp_ops.ops()                            # loads libopensplat_b200_ops.so
+def _train_mirror():
+    """The same loop (same problem, seed and schedule) over opensplat_b200.model.GaussianModel."""
     from opensplat_b200.densify import RefineConfig
     from opensplat_b200.model import Camera, GaussianModel
-    torch.ops.load_library(LIB)
     p, c2w, gts, (fx, fy, cx, cy), H, W = make_problem()
-    steps, seed, ssim_w, sh_int = 34, 11, 0.2, 8
-    cfg = RefineConfig(refine_every=10, warmup_length=15, reset_alpha_every=30, densify_grad_thresh=2e-5,
-                       densify_size_thresh=0.05, stop_screen_size_at=4000, split_screen_size=0.05, max_steps=200,
-                       num_cameras=3)
-    params = [torch.from_numpy(p[x]).to(DEV) for x in PARAM_NAMES]
-    out = torch.ops.opensplat_b200_model.train(
-        params, torch.from_numpy(c2w), torch.from_numpy(gts), fx, fy, cx, cy, H, W, 1, steps, ssim_w, seed, sh_int,
-        cfg.num_cameras, cfg.refine_every, cfg.warmup_length, cfg.reset_alpha_every, cfg.densify_grad_thresh,
-        cfg.densify_size_thresh, cfg.stop_screen_size_at, cfg.split_screen_size, cfg.max_steps)
-    ref_loss, ref_cnt, ref_rgb = out[0].numpy(), out[1].numpy(), out[2]
-    ref_params = dict(zip(PARAM_NAMES, out[3:9]))
-    assert np.isfinite(ref_loss).all() and ref_loss[18] < ref_loss[0]            # it trains
-    assert ref_cnt[18] == len(p["means"]) and ref_cnt[19] != ref_cnt[18] and ref_cnt[29] != ref_cnt[28]  # 2 refinements
-
-    model = GaussianModel({k: torch.from_numpy(v) for k, v in p.items()}, cfg, sh_degree_interval=sh_int, device=DEV)
+    model = GaussianModel({k: torch.from_numpy(v) for k, v in p.items()}, RefineConfig(**TRAIN_REFINE),
+                          sh_degree_interval=TRAIN_SH_INTERVAL, device=DEV)
     cams = [Camera(W, H, fx, fy, cx, cy, c2w[v]) for v in range(len(c2w))]
     gt_dev = torch.from_numpy(gts).to(DEV)
-    torch.manual_seed(seed)
+    torch.manual_seed(TRAIN_SEED)
     losses, counts, rgb = [], [], None
-    for step in range(1, steps + 1):
+    for step in range(1, TRAIN_STEPS + 1):
         v = (step - 1) % len(cams)
         model.optimizers_zero_grad()
         rgb = model.forward(cams[v], step)
-        loss = model.main_loss(rgb, gt_dev[v], ssim_w)
+        loss = model.main_loss(rgb, gt_dev[v], TRAIN_SSIM_WEIGHT)
         loss.backward()
         losses.append(float(loss.detach()))
         model.optimizers_step()
         model.schedulers_step(step)
         model.after_train(step)
         counts.append(model.means.shape[0])
-    losses, counts = np.array(losses), np.array(counts)
+    return np.array(losses), np.array(counts), rgb.detach(), {k: getattr(model, k).detach() for k in PARAM_NAMES}
+
+
+def _assert_follows(run, ref):
+    (losses, counts, rgb, params), (ref_loss, ref_cnt, ref_rgb, ref_params, rows) = run, ref
     assert np.abs(losses[:20] - ref_loss[:20]).max() <= 5e-5, np.abs(losses[:20] - ref_loss[:20]).max()
     assert np.abs(counts - ref_cnt).max() <= 0.02 * ref_cnt.max(), (counts[[19, 29]], ref_cnt[[19, 29]])
     assert np.abs(losses - ref_loss).max() <= 5e-3, np.abs(losses - ref_loss).max()
     if np.array_equal(counts, ref_cnt):          # identical discrete decisions: the parameter sets line up row by row
         for k in PARAM_NAMES:
-            a, b = getattr(model, k).detach(), ref_params[k]
-            assert a.shape == b.shape
+            a, b = params[k], ref_params[k]
+            assert a.shape[0] == ref_cnt[-1] and a.shape[1:] == b.shape[1:], k
+            a = a.index_select(0, rows)
             assert float((a - b).abs().max()) <= 2e-3 * (1.0 + float(b.abs().max())), k
-        assert float((rgb.detach() - ref_rgb).abs().max()) <= 2e-2
-
-
-@pytest.mark.skipif(not os.path.exists(LIB), reason="libopensplat_model_b200.so not built (needs /root/reference at build time)")
-def test_reference_training_loop_with_cpp_fused_opt_ins_follows_the_unchanged_one():
-    """SURVEY 8f row 1 from C++: the reference's loop with the bodies of Model::forward / Model::mainLoss swapped for
-    gsb::modelForward (ProjectGaussiansActivated -> SphericalHarmonicsRgb -> RasterizeGaussiansClamped) and
-    gsb::MainLoss (csrc/ops/fused_extras.hpp; driver op train_fused) against the UNCHANGED model.cpp on the same
-    operators: same losses to rounding, same refinement decisions; optimizers / schedulers / afterTrain are the
-    reference's own code in both runs."""
-    from opensplat_b200 import cpp_ops
-    cpp_ops.ops()
-    from opensplat_b200.densify import RefineConfig
-    torch.ops.load_library(LIB)
-    p, c2w, gts, (fx, fy, cx, cy), H, W = make_problem()
-    steps, seed, ssim_w, sh_int = 34, 11, 0.2, 8
-    cfg = RefineConfig(refine_every=10, warmup_length=15, reset_alpha_every=30, densify_grad_thresh=2e-5,
-                       densify_size_thresh=0.05, stop_screen_size_at=4000, split_screen_size=0.05, max_steps=200,
-                       num_cameras=3)
-    outs = []
-    for op in (torch.ops.opensplat_b200_model.train, torch.ops.opensplat_b200_model.train_fused):
-        params = [torch.from_numpy(p[x]).to(DEV) for x in PARAM_NAMES]
-        out = op(params, torch.from_numpy(c2w), torch.from_numpy(gts), fx, fy, cx, cy, H, W, 1, steps, ssim_w, seed,
-                 sh_int, cfg.num_cameras, cfg.refine_every, cfg.warmup_length, cfg.reset_alpha_every,
-                 cfg.densify_grad_thresh, cfg.densify_size_thresh, cfg.stop_screen_size_at, cfg.split_screen_size,
-                 cfg.max_steps)
-        outs.append((out[0].numpy(), out[1].numpy(), out[2], dict(zip(PARAM_NAMES, out[3:9]))))
-    (ref_loss, ref_cnt, ref_rgb, ref_p), (loss, cnt, rgb, par) = outs
-    assert ref_cnt[19] != ref_cnt[18] and ref_cnt[29] != ref_cnt[28]                # two refinements happened
-    assert np.abs(loss[:20] - ref_loss[:20]).max() <= 5e-5, np.abs(loss[:20] - ref_loss[:20]).max()
-    assert np.abs(cnt - ref_cnt).max() <= 0.02 * ref_cnt.max(), (cnt[[19, 29]], ref_cnt[[19, 29]])
-    assert np.abs(loss - ref_loss).max() <= 5e-3, np.abs(loss - ref_loss).max()
-    if np.array_equal(cnt, ref_cnt):
-        for k in PARAM_NAMES:
-            assert float((par[k] - ref_p[k]).abs().max()) <= 2e-3 * (1.0 + float(ref_p[k].abs().max())), k
         assert float((rgb - ref_rgb).abs().max()) <= 2e-2
+
+
+def test_reference_model_cpp_unchanged_trains_on_b200_backend_and_mirror_follows():
+    _assert_follows(_train_mirror(), _reference_run())
+
+
+def _cpp_model_forward(model, cam, step):
+    """What Model::forward becomes when a maintainer opts in (INTEGRATION.md; tests/native/model_driver.cpp's fused
+    branch): gsb::modelForward on the down-scaled camera, xys / radii / image size kept for afterTrain."""
+    sf = float(model.get_downscale_factor(step))
+    h, w = int(float(cam.height) / sf), int(float(cam.width) / sf)
+    rgb, xys, radii = torch.ops.opensplat_b200_test.model_forward(
+        model.means, model.scales, model.quats, model.featuresDc, model.featuresRest, model.opacities,
+        model.backgroundColor, cam.camToWorld, cam.fx / sf, cam.fy / sf, cam.cx / sf, cam.cy / sf, h, w,
+        min(step // model.shDegreeInterval, model.shDegree))
+    model.xys, model.radii, model.lastHeight, model.lastWidth = xys, radii, h, w
+    return rgb
+
+
+def test_cpp_model_forward_and_main_loss_opt_ins_follow_the_reference_training_loop(monkeypatch):
+    """SURVEY 8f row 1 from C++: gsb::modelForward (host-side camera matrices, tile bounds, background early return,
+    then ProjectGaussiansActivated -> SphericalHarmonicsRgb -> RasterizeGaussiansClamped) and gsb::MainLoss
+    (csrc/ops/fused_extras.hpp) as the forward and loss of the mirror's training loop (its Adam, schedule and
+    afterTrain) follow the reference's UNCHANGED model.cpp loop on the same operators (golden): same losses to
+    rounding, same refinement decisions."""
+    from opensplat_b200 import cpp_ops, model as model_mod
+    from opensplat_b200.model import Camera, GaussianModel
+    o = cpp_ops.ops()
+    torch.ops.load_library(os.path.join(ROOT, "tests", "native", "_build", "libopensplat_b200_test_ops.so"))
+
+    # no Gaussian in view (camera turned away from the scene): the background, as Model::forward returns it
+    p, c2w, _, (fx, fy, cx, cy), H, W = make_problem()
+    away = c2w[len(c2w) // 2].copy()
+    away[:3, :3] = away[:3, :3] @ np.diag([-1.0, 1.0, -1.0]).astype(np.float32)
+    m = GaussianModel({k: torch.from_numpy(v) for k, v in p.items()}, device=DEV)
+    cam = Camera(W, H, fx, fy, cx, cy, away)
+    m.backgroundColor = torch.tensor([0.25, 0.5, 0.75], device=DEV)
+    rgb = _cpp_model_forward(m, cam, 1)
+    assert int(m.radii.sum()) == 0 and rgb.shape == (m.lastHeight, m.lastWidth, 3)
+    assert torch.equal(rgb, m.backgroundColor.repeat(m.lastHeight, m.lastWidth, 1))
+
+    monkeypatch.setattr(GaussianModel, "forward", _cpp_model_forward)
+    monkeypatch.setattr(model_mod.ops, "MainLoss", types.SimpleNamespace(apply=o.main_loss))
+    _assert_follows(_train_mirror(), _reference_run())
 
 
 def test_gaussian_model_save_matches_reference_writer(tmp_path):

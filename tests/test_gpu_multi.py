@@ -3,7 +3,7 @@ fused exchange launch vs sh_backward + one NCCL all-reduce of the flat buffer, r
 steps, and both again after a lock-step change of the Gaussian count (odd N).
  * world size 1 runs everywhere (symmetric memory, re-binding of the gradient buffer, both CTA roles of the launch,
    resize) -- the driver's 1-GPU box included;
- * world size 2 needs two devices (skipped otherwise; run under `gpurun --gpus 2`), once with the NVSwitch multimem
+ * world size 2 needs two devices (skipped otherwise), once with the NVSwitch multimem
    all-reduce role and once with the peer-pointer one."""
 import os
 import subprocess
@@ -34,7 +34,7 @@ def test_fused_exchange_world1_end_to_end():
 
 def test_fused_exchange_matches_nccl_allreduce_2gpu():
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run under `gpurun --gpus 2`)")
+        pytest.skip("needs 2 GPUs")
     out = _run(2, 29533)
     out2 = _run(2, 29535, {"GSB_EXCHANGE_MULTICAST": "0"})
     assert "multicast=False" in out2

@@ -50,3 +50,31 @@ def scene_edit_inputs(n, sh_bases, seed, max_dim=640):
         v_xy[radii <= 0] = 0
         steps.append((v_xy, radii))
     return p, m, v, steps
+
+
+# ---- the short training run of tests/test_gpu_model.py (tests/golden/make_golden_b200.py records the reference's) ----
+TRAIN_STEPS, TRAIN_SEED, TRAIN_SSIM_WEIGHT, TRAIN_SH_INTERVAL = 34, 11, 0.2, 8
+TRAIN_REFINE = dict(num_cameras=3, refine_every=10, warmup_length=15, reset_alpha_every=30, densify_grad_thresh=2e-5,
+                    densify_size_thresh=0.05, stop_screen_size_at=4000, split_screen_size=0.05, max_steps=200)
+
+
+def make_problem(n=4000, V=3, H=96, W=128, k=4, seed=5):
+    rng = np.random.default_rng(seed)
+    f = np.float32
+    p = {
+        "means": (rng.uniform(-1, 1, (n, 3)) * np.array([1.6, 1.2, 0.5])).astype(f),
+        "scales": np.log(rng.uniform(0.02, 0.12, (n, 3))).astype(f),
+        "quats": rng.standard_normal((n, 4)).astype(f),
+        "featuresDc": rng.uniform(-1.5, 1.5, (n, 3)).astype(f),
+        "featuresRest": (rng.standard_normal((n, k - 1, 3)) * 0.1).astype(f),
+        "opacities": rng.uniform(-2.0, 1.0, (n, 1)).astype(f),
+    }
+    c2w = np.tile(np.eye(4, dtype=f), (V, 1, 1))
+    for v in range(V):                       # OpenGL-style poses on a circle of radius 4, looking at the origin
+        a = 0.25 * (v - (V - 1) / 2)
+        c2w[v, :3, :3] = np.array([[np.cos(a), 0, -np.sin(a)], [0, 1, 0], [np.sin(a), 0, np.cos(a)]], dtype=f)
+        c2w[v, :3, 3] = np.array([-4.0 * np.sin(a), 0.0, 4.0 * np.cos(a)], dtype=f)
+    yy, xx = np.mgrid[0:H, 0:W]
+    gts = np.stack([np.stack([0.5 + 0.5 * np.sin(0.07 * xx + v), 0.5 + 0.5 * np.cos(0.05 * yy - v),
+                              0.5 + 0.25 * np.sin(0.03 * (xx + yy))], -1) for v in range(V)]).astype(f)
+    return p, c2w, gts, (0.9 * W, 0.9 * W, W / 2.0, H / 2.0), H, W

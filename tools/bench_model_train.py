@@ -55,7 +55,8 @@ def main():
     from opensplat_b200.densify import RefineConfig
     from opensplat_b200.model import Camera, GaussianModel, PARAM_NAMES
     cpp_ops.ops()
-    torch.ops.load_library(os.path.join(ROOT, "tests", "native", "_build", "libopensplat_model_b200.so"))
+    from oracle.build_model_b200 import OUT as MODEL_LIB
+    torch.ops.load_library(MODEL_LIB)
     W, H = a.W, a.H
     p, c2w, (fx, fy, cx, cy) = model_scene(a.n, W, H)
     gts = torch.rand(1, H, W, 3)
